@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU algorithm (oracle port)
+    python bench.py --steps K --dump-outputs DIR             # + the outputs of the last timed step of every leg as DIR/*.npy
 
 Primary line  = ORB keypoints/s, BASELINE configs[1]: 640x480, 8 levels, 1000 kps/frame, batch of 64 frames / GPU.
 `secondary`   = LM iterations/s, BASELINE configs[3]: 50 KF / 5000 landmarks / ~29k edges, Huber, 10 LM iterations.
@@ -20,6 +21,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -106,6 +108,25 @@ def matcher_frames():
         a = synth.orb_frame(2000 + k)
         imgs += [a, np.roll(a, (3 + k % 3, -5 + k % 4), axis=(0, 1))]
     return np.stack(imgs)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def kp_columns(kps):
+    """[..., 7] float32 columns (x, y, size, angle, response, octave, class_id) of KP_DTYPE records; exact for the int fields."""
+    return np.stack([kps[f].astype(np.float32) for f in kps.dtype.names], axis=-1)
+
+
+def write_dump(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, float32 or float64 only."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def dist_env():
@@ -265,6 +286,18 @@ def run_ours(args):
         orb_join()
         e1.record(stream)
         barrier()
+    dump = {}
+    if args.dump_outputs:
+        # what the last timed step handed its caller: per-frame counts, keypoints and descriptors of the 64-frame batch; the
+        # slots past a frame's count are not written by the extractor and are zeroed here
+        last = args.steps - 1
+        kq, dq = outs2[last % inflight]
+        n = d_counts[last].cpu().numpy()
+        valid = (np.arange(NFEAT)[None, :] < n[:, None])[..., None]
+        kp = kq.cpu().numpy().view(_capi.KP_DTYPE).reshape(BATCH, NFEAT)
+        dump["orb_counts"] = n.astype(np.float32)
+        dump["orb_keypoints"] = np.where(valid, kp_columns(kp), 0).astype(np.float32)
+        dump["orb_descriptors"] = np.where(valid, dq.cpu().numpy().reshape(BATCH, NFEAT, 32), 0).astype(np.float32)
     kp_total = d_counts[:args.steps].sum()
     orb_ms = max_over_ranks(e0.elapsed_time(e1))
     # the same K steps strictly one after the other on one context / stream (what a single se2gpu_orb handle delivers)
@@ -368,7 +401,7 @@ def run_ours(args):
     # pageable caller buffers (input and outputs): staged through the library's page-locked buffers
     page_in = [np.array(host_batches[r].numpy(), copy=True) for r in range(min(NROT, 3))]
     kps_p = np.zeros(BATCH * NFEAT, _capi.KP_DTYPE); desc_p = np.zeros(BATCH * NFEAT * 32, np.uint8); counts_p = np.zeros(BATCH, np.int32)
-    pg_steps = min(e2e_steps, 8)
+    pg_steps = e2e_steps
     t0 = time.perf_counter()
     totp = 0
     for k in range(pg_steps):
@@ -429,6 +462,12 @@ def run_ours(args):
         match_step(k)
     m1.record(stream)
     barrier()
+    if args.dump_outputs:       # the last timed pair: vnMatches12, the updated vbPrevMatched and the number of matches
+        pi = (msteps - 1) % MATCH_PAIRS
+        n1 = int(m_counts[2 * pi].item())
+        dump["matcher_matches12"] = m_out[pi, :n1].cpu().numpy().astype(np.float32)
+        dump["matcher_prev_matched"] = m_prev[:2 * n1].cpu().numpy().reshape(n1, 2)
+        dump["matcher_nmatches"] = m_nm[pi:pi + 1].cpu().numpy().astype(np.float32)
     match_ms = max_over_ranks(m0.elapsed_time(m1))
     match_launches = lib.se2gpu_launch_count() - ml0
     match_value = sum_over_ranks(float(msteps)) / (match_ms * 1e-3)
@@ -530,6 +569,9 @@ def run_ours(args):
         iters += n
     b1.record(stream)
     barrier()
+    if args.dump_outputs:       # the last optimize(): estimates and the chi2 after each iteration
+        dump["ba_poses"], dump["ba_points"] = ba.get()
+        dump["ba_chi2"] = np.ascontiguousarray(st["chi2_after"], np.float64)
     ba_ms = max_over_ranks(b0.elapsed_time(b1))
     ba_launches = lib.se2gpu_launch_count() - bl0
     bprof = ba.profile_read()
@@ -577,7 +619,7 @@ def run_ours(args):
         prob5 = synth.ba_config("C5")
         ba5 = LocalBA.from_problem(prob5, device=local_rank, rank=rank, world=world, allreduce=allreduce if world > 1 else None, stream=sptr)
         ba5.optimize(C5_ITERS)
-        c5_steps = max(2, min(args.steps, 6))
+        c5_steps = args.steps
         barrier()
         ba5.profile(True)
         c5l0 = lib.se2gpu_launch_count()
@@ -591,6 +633,9 @@ def run_ours(args):
             it5 += n5
         c1.record(stream)
         barrier()
+        if args.dump_outputs:
+            dump["c5_poses"], dump["c5_points"] = ba5.get()
+            dump["c5_chi2"] = np.ascontiguousarray(st5["chi2_after"], np.float64)
         c5_ms = max_over_ranks(c0.elapsed_time(c1))
         c5_launches = lib.se2gpu_launch_count() - c5l0
         c5prof = {g: v for g, v in ba5.profile_read().items() if v[1] > 0}
@@ -667,6 +712,8 @@ def run_ours(args):
                 t1 = time.perf_counter(); n5c, _ = o5.optimize(3); dt5 = time.perf_counter() - t1
                 line["tertiary"]["cpu_baseline"] = {"value": n5c / dt5, "unit": "LM iterations/s", "cores": 1, "kind": "port", "host_cores": os.cpu_count(),
                                                     "sample": "1 x optimize(3) of the same window, single thread (skyline Cholesky)"}
+        if args.dump_outputs:       # rank 0's outputs
+            write_dump(args.dump_outputs, dump)
         _OUT.write(json.dumps(line) + "\n"); _OUT.flush()
     if world > 1:
         dist.destroy_process_group()
@@ -692,9 +739,12 @@ def cpu_baselines():
     # and therefore the keypoints, are the same)
     try:
         import ctypes as C
-        subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "native", "CXX=g++"], check=True, timeout=300,
-                       stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-        N = C.CDLL(os.path.join(ROOT, "oracle", "liboracle_native.so"))
+        # built for this host's CPU at run time, in a temporary directory: the benchmark writes nothing into the tree
+        with tempfile.TemporaryDirectory() as tmp:
+            native = os.path.join(tmp, "liboracle_native.so")
+            subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "native", "CXX=g++", f"NATIVE_LIB={native}"], check=True,
+                           timeout=300, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            N = C.CDLL(native)
         N.orb_oracle_create.restype = C.c_void_p
         N.orb_oracle_create.argtypes = [C.c_int, C.c_float, C.c_int, C.c_int]
         N.orb_oracle_extract.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
@@ -749,13 +799,19 @@ def main():
     _OUT = _reserve_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every leg (the matcher leg times one pass over its pairs per step)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--quick", action="store_true", help="profiling runs: skip the CPU baseline and the e2e legs")
     ap.add_argument("--orb-inflight", type=int, default=1, help="64-frame batches in flight in the device-resident ORB leg (2 = two extractor contexts / streams; measured +1.7 %: the kernels already fill the machine)")
     ap.add_argument("--no-c5", action="store_true", help="skip the BASELINE configs[4] leg (2000 KF / 50k landmarks; ~20 s of host-side synthesis)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of every leg as DIR/<name>.npy "
+                                                          "(float32 / float64; inputs are seeded, so two builds can be compared file by file)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repo's CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
